@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the OCR forward hot path on B200, one JSON line per run (rank 0).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`; the default is the one the headline metric is quoted on):
 
@@ -284,6 +284,43 @@ def mgp_decoded_chars(ids):
     return int(first.sum())
 
 
+def dump_outputs(out, w, outdir):
+    """Write what one batch of the timed path returned to its caller as `outdir/<name>.npy`: token ids as float64 (exact),
+    probabilities as float32.  Per-page sequences are padded with -1 to the workload's maximum length, so every run of a
+    workload writes the same shapes and two builds can be compared array for array (well under 64 MB for every workload)."""
+    import numpy as np
+    B = out[0].shape[1] if w['kind'] == 'mgp' else len(out)
+    if w['kind'] == 'mgp':
+        ids, prob = out
+        arrays = {'ids': ids.numpy().astype(np.float64), 'probs': prob.numpy().astype(np.float32)}
+    elif w['points_only']:
+        P = w['pt_len']
+        n = np.zeros(B)
+        tok, pr = np.full((B, P), -1.0), np.full((B, P), -1.0, dtype=np.float32)
+        for b, (t, p) in enumerate(out):
+            n[b] = t.numel()
+            tok[b, :t.numel()], pr[b, :p.numel()] = t.numpy(), p.numpy()
+        arrays = {'n_tokens': n, 'pt': tok, 'pt_probs': pr}
+    else:
+        maxi = w['pt_len'] // 2
+        n = np.zeros(B)
+        pt, poly, rec = np.full((B, maxi, 2), -1.0), np.full((B, maxi, 32), -1.0), np.full((B, maxi, REC_LEN), -1.0)
+        prob = np.full((B, maxi, REC_LEN), -1.0, dtype=np.float32)
+        for b, o in enumerate(out):
+            if o is None:          # no point decoded on this page
+                continue
+            (p, q, r), (pr,) = o
+            k = p.numel() // 2
+            n[b] = k
+            pt[b, :k], poly[b, :k] = p.numpy().reshape(k, 2), q.numpy().reshape(k, 32)
+            rec[b, :k], prob[b, :k] = r.numpy()[0], pr.numpy()
+        arrays = {'n_instances': n, 'pt': pt, 'poly': poly, 'rec': rec, 'rec_probs': prob}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    os.makedirs(outdir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(outdir, k + '.npy'), a)
+
+
 def self_check_omni(out0):
     """Page 0 of rank 0 (page seed 1000) against the reference's own output (tests/golden/omni_config2_page0.npz,
     written by oracle/gen_golden.py config2 from the unmodified reference).  Sequences that leave the reference are
@@ -325,8 +362,14 @@ def main():
                     'the compute threads do not wait (dist.CollectiveLane; measured: no gain at 2 GPUs, lower e2e)')
     ap.add_argument('--watchdog-s', type=float, default=600.0, help='a timed phase that takes longer dumps every host '
                     'thread\'s stack to stderr and exits non-zero (a hung collective must not burn the GPU box)')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR', help='after the timed steps, write what the last timed '
+                    'step returned (rank 0\'s batch) as DIR/<name>.npy, for output-for-output comparison of two builds')
     ap.add_argument('--cpu-child', nargs=3, default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of the GPU arm (--impl ours)')
     if args.cpu_child:
         return _cpu_child(args.cpu_child[0], int(args.cpu_child[1]), int(args.cpu_child[2]))
     if args.impl == 'reference':
@@ -545,6 +588,8 @@ def main():
         sampler.start()
     ms_total, launches, last = timed(step_resident, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last[(args.steps - 1) % C_][0], w, args.dump_outputs)   # step s ran on context s % C
     ms_e2e, _, last_e2e = timed(step_e2e, args.steps, max(3, args.warmup // 2))
 
     out0, gathered0 = last[0]

@@ -53,6 +53,36 @@ def test_mgp_decoded_chars_counts_tokens_before_eos():
     assert b.mgp_decoded_chars(ids) == 3 + 26
 
 
+def test_dump_outputs_writes_fixed_shape_float_arrays(tmp_path):
+    """bench.py --dump-outputs: per workload kind, what the timed path returns is written as float32 / float64 .npy files
+    of fixed shape (ragged per-page sequences padded with -1), with the ids and probabilities unchanged."""
+    import numpy as np
+    import torch
+    b = _bench()
+    L, maxi = b.REC_LEN, b.WORKLOADS['omni']['pt_len'] // 2
+    page = lambda n: ([torch.arange(2 * n).reshape(1, -1), torch.arange(32 * n).reshape(1, -1) + 7,
+                       torch.arange(n * L).reshape(1, n, L) + 1000], [torch.rand(n, L)])
+    omni = [page(3), None, page(maxi)]
+    b.dump_outputs(omni, b.WORKLOADS['omni'], str(tmp_path / 'omni'))
+    d = {k: np.load(tmp_path / 'omni' / f'{k}.npy') for k in ('n_instances', 'pt', 'poly', 'rec', 'rec_probs')}
+    assert d['n_instances'].tolist() == [3, 0, maxi]
+    assert d['pt'].shape == (3, maxi, 2) and d['poly'].shape == (3, maxi, 32) and d['rec'].shape == (3, maxi, L)
+    assert d['rec_probs'].dtype == np.float32 and all(d[k].dtype == np.float64 for k in ('n_instances', 'pt', 'poly', 'rec'))
+    assert np.array_equal(d['poly'][0, :3].reshape(-1), omni[0][0][1].numpy()[0]) and (d['poly'][0, 3:] == -1).all()
+    assert (d['pt'][1] == -1).all() and np.array_equal(d['rec'][2], omni[2][0][2].numpy()[0])
+    assert np.array_equal(d['rec_probs'][0, :3], omni[0][1][0].numpy())
+    P = b.WORKLOADS['table']['pt_len']
+    pts = [(torch.arange(5), torch.rand(5)), (torch.arange(P), torch.rand(P))]
+    b.dump_outputs(pts, b.WORKLOADS['table'], str(tmp_path / 'table'))
+    tok, pr = np.load(tmp_path / 'table' / 'pt.npy'), np.load(tmp_path / 'table' / 'pt_probs.npy')
+    assert tok.shape == pr.shape == (2, P) and np.load(tmp_path / 'table' / 'n_tokens.npy').tolist() == [5, P]
+    assert np.array_equal(tok[0, :5], np.arange(5)) and (tok[0, 5:] == -1).all() and np.array_equal(pr[1], pts[1][1].numpy())
+    ids, prob = torch.randint(0, 50, (3, 4, 27), dtype=torch.int32), torch.rand(3, 4, 27)
+    b.dump_outputs((ids, prob), b.WORKLOADS['mgpstr'], str(tmp_path / 'mgp'))
+    assert np.array_equal(np.load(tmp_path / 'mgp' / 'ids.npy'), ids.numpy())
+    assert np.array_equal(np.load(tmp_path / 'mgp' / 'probs.npy'), prob.numpy())
+
+
 def _plan(npairs, nkb, num_sms, ctas_per_sm):
     """cross_attn_mq_plan (csrc/xattn.cu)."""
     nb = npairs * nkb
