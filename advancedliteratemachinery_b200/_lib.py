@@ -71,6 +71,10 @@ SIGNATURES = {
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     'alm_omni_decode_points': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(DecodeCfg), C.c_void_p, C.c_void_p,
                                          C.c_void_p]),
+    'alm_omni_decode_prompted': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(DecodeCfg), C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    'alm_omni_decode_points_prompted': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(DecodeCfg),
+                                                  C.c_void_p, C.c_void_p, C.c_void_p]),
     'alm_omni_decode_logits': (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     'alm_omni_vocab': (C.c_int, [C.c_void_p]),
     'alm_omni_last_timing': (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_float)]),

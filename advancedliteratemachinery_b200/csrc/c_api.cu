@@ -659,6 +659,22 @@ int alm_omni_decode_points(alm_ctx* h, const int64_t* pt_prompt, int n_prompt, c
   });
 }
 
+int alm_omni_decode_prompted(alm_ctx* h, const int64_t* prompts, int R, int n_prompt, const alm_decode_cfg* cfg,
+                             int32_t* n_inst, int64_t* pt, int64_t* poly, int64_t* rec, float* rec_prob) {
+  return guarded(h, [&] {
+    ALM_REQUIRE(prompts && cfg && n_inst && pt && poly && rec && rec_prob, ALM_ERR_INVALID, "null argument");
+    omni_decode_prompted(&h->c, prompts, R, n_prompt, *cfg, n_inst, pt, poly, rec, rec_prob);
+  });
+}
+
+int alm_omni_decode_points_prompted(alm_ctx* h, const int64_t* prompts, int R, int n_prompt, const alm_decode_cfg* cfg,
+                                    int32_t* n_tok, int64_t* pt_tokens, float* pt_probs) {
+  return guarded(h, [&] {
+    ALM_REQUIRE(prompts && cfg && n_tok && pt_tokens, ALM_ERR_INVALID, "null argument");
+    omni_decode_points_prompted(&h->c, prompts, R, n_prompt, *cfg, n_tok, pt_tokens, pt_probs);
+  });
+}
+
 int alm_omni_decode_logits(alm_ctx* h, int image, int kind, const int64_t* seq, int n_seq, int len, float* logits) {
   return guarded(h, [&] {
     ALM_REQUIRE(seq && logits, ALM_ERR_INVALID, "null argument");

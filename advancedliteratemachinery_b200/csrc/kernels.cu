@@ -457,7 +457,7 @@ softmax_rows_kernel(const float* __restrict__ s, long lds, int n, const uint8_t*
 
 
 // ---------------------------------------------------------------------------------------------
-// Skinny fp32 linear for the single-sequence-per-image decode (M <= 32 rows): out[m, n] = act(x[m,:].W[n,:] + b[n])
+// Skinny fp32 linear for the point-loop decode (M <= 64 rows): out[m, n] = act(x[m,:].W[n,:] + b[n])
 // (+ resid[m, n]).  One warp per output column streams its fp32 weight row once (coalesced float4) while the few
 // activation rows come from L1; a tensor-core tile would be > 90 % padding here and the op is latency-bound anyway.
 // Weights stay exact fp32, so this path is closer to the reference than the split-bf16 GEMM.
@@ -467,18 +467,27 @@ softmax_rows_kernel(const float* __restrict__ s, long lds, int n, const uint8_t*
 // the latency-bound point loop) with exactly the arithmetic and summation order of gather_ln_kernel<4>, then adds the
 // query position embedding `pos` for the output columns below pos_split (q | k of the packed self-attention projection;
 // everything for the cross-attention query).
-template <int MR, int NW>  // MR = row capacity (8/16/32), NW = K / 128 float4 slices of the weight row per lane
-__global__ void __launch_bounds__(128)
-gemv_rows_kernel(const float* __restrict__ x, const float* __restrict__ x2, int n_split, long ldx,
+//
+// The 64-row variant (up to 64 live sequences: several window prompts per page in the point loop) keeps every row's
+// arithmetic of the 32-row one -- each lane still accumulates one row in the same lane-strided float4 order over K and the
+// row is reduced by the same warp_sum -- so a row's result does not depend on how many rows share the launch.  Lane l
+// writes rows l and l + 32.  Its K > 512 launches stage 256-float chunks (64 x 2 x 256 fp32 = 128 KB double-buffered,
+// where 512-float chunks would need 256 KB): chunk c of 512 floats is chunks 2c, 2c + 1 of 256, so the per-lane order of
+// the fused multiply-adds is unchanged.
+template <int MR, int NW>  // MR = row capacity (8/16/32/64), NW = K / 128 float4 slices of the weight row per lane
+__device__ __forceinline__ void
+gemv_rows_body(const float* __restrict__ x, const float* __restrict__ x2, int n_split, long ldx,
                  const float* __restrict__ W, const float* __restrict__ bias, const float* __restrict__ resid, long ldr,
                  float* __restrict__ out, long ldo, int M, int N, int K, int act, const float* __restrict__ ln_g,
                  const float* __restrict__ ln_b, float ln_eps, const float* __restrict__ pos, int pos_split) {
   // activation rows, staged in K-chunks of <= 512 floats (double-buffered when K > 512): at most 64 KB for 16 rows,
   // so this kernel co-resides with the HBM-bound attention CTAs of the other in-flight decode streams
   extern __shared__ __align__(16) float sx[];
-  constexpr int NC = (NW + 3) / 4;          // chunks
-  constexpr int NWC = NW < 4 ? NW : 4;      // float4 slices per lane and chunk
-  const int KC = NC == 1 ? K : 512;         // chunk width (floats)
+  constexpr int CW = (MR > 32 && NW > 4) ? 256 : 512;  // chunk width when K > 512 (floats)
+  constexpr int SPC = CW / 128;             // float4 slices per lane of a full chunk
+  constexpr int NC = (NW + SPC - 1) / SPC;  // chunks
+  constexpr int NWC = NW < SPC ? NW : SPC;  // float4 slices per lane and chunk
+  const int KC = NC == 1 ? K : CW;          // chunk width (floats)
   const int n = blockIdx.x * 4 + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   const float* xin = (blockIdx.x * 4 < n_split) ? x : x2;  // columns [0, n_split) read x, the rest x2 (fused q|k|v)
@@ -495,9 +504,12 @@ gemv_rows_kernel(const float* __restrict__ x, const float* __restrict__ x2, int 
   };
   stage(0, 0);  // every 16-byte copy of the chunk is in flight at once: one memory round trip however many rows
   // the whole weight row of this column is requested up front (NW independent 16-byte loads per lane = one
-  // round trip), overlapping the activation staging
+  // round trip), overlapping the activation staging.  The 64-row kernel, whose 64 accumulators already take the
+  // registers, requests each chunk's slices at the top of that chunk instead (same values, same order of use).
+  constexpr bool PRELOAD = MR <= 32;
   float4 w[NW];
-  if (n < N) {
+  if (!PRELOAD) {
+  } else if (n < N) {
     const float* wrow = W + static_cast<long>(n) * K;
 #pragma unroll
     for (int i = 0; i < NW; ++i) {
@@ -513,6 +525,14 @@ gemv_rows_kernel(const float* __restrict__ x, const float* __restrict__ x2, int 
   for (int m = 0; m < MR; ++m) acc[m] = 0.f;
 #pragma unroll
   for (int c = 0; c < NC; ++c) {
+    if (!PRELOAD) {
+#pragma unroll
+      for (int i = 0; i < NWC; ++i) {
+        const int k0 = ((c * SPC + i) * 32 + lane) * 4;
+        w[c * SPC + i] = (n < N && k0 < K) ? *reinterpret_cast<const float4*>(W + static_cast<long>(n) * K + k0)
+                                           : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
+    }
     if (c + 1 < NC) {
       stage(c + 1, (c + 1) & 1);
       asm volatile("cp.async.wait_group 1;" ::: "memory");
@@ -567,7 +587,7 @@ gemv_rows_kernel(const float* __restrict__ x, const float* __restrict__ x2, int 
           const int kk = (i * 32 + lane) * 4;
           if (c * KC + kk < K) {
             const float4 a = *reinterpret_cast<const float4*>(xs + m * KC + kk);
-            const float4 ww = w[c * 4 + i];
+            const float4 ww = w[c * SPC + i];
             acc[m] = fmaf(a.x, ww.x, acc[m]); acc[m] = fmaf(a.y, ww.y, acc[m]);
             acc[m] = fmaf(a.z, ww.z, acc[m]); acc[m] = fmaf(a.w, ww.w, acc[m]);
           }
@@ -577,20 +597,44 @@ gemv_rows_kernel(const float* __restrict__ x, const float* __restrict__ x2, int 
     if (c + 2 < NC) __syncthreads();  // the buffer is refilled two chunks later
   }
   if (n >= N) return;
-  float mine = 0.f;
+  constexpr int RPL = (MR + 31) / 32;  // rows written per lane
+  float mine[RPL];
+#pragma unroll
+  for (int j = 0; j < RPL; ++j) mine[j] = 0.f;
 #pragma unroll
   for (int m = 0; m < MR; ++m) {
     const float v = warp_sum(acc[m]);
-    if (lane == m) mine = v;
+    if (lane == (m & 31)) mine[m >> 5] = v;
   }
-  if (lane < M && lane < MR) {
-    float v = mine + (bias ? bias[n] : 0.f);
-    if (act == ACT_GELU) v = 0.5f * v * (1.0f + erff(v * 0.70710678118654752440f));
-    else if (act == ACT_RELU) v = fmaxf(v, 0.f);
-    if (resid) v += resid[lane * ldr + n];
-    out[lane * ldo + n] = v;
+#pragma unroll
+  for (int j = 0; j < RPL; ++j) {
+    const int row = j * 32 + lane;
+    if (row < M && row < MR) {
+      float v = mine[j] + (bias ? bias[n] : 0.f);
+      if (act == ACT_GELU) v = 0.5f * v * (1.0f + erff(v * 0.70710678118654752440f));
+      else if (act == ACT_RELU) v = fmaxf(v, 0.f);
+      if (resid) v += resid[row * ldr + n];
+      out[row * ldo + n] = v;
+    }
   }
 }
+
+#define ALM_GEMV_PARAMS                                                                                              \
+  const float *__restrict__ x, const float *__restrict__ x2, int n_split, long ldx, const float *__restrict__ W,    \
+      const float *__restrict__ bias, const float *__restrict__ resid, long ldr, float *__restrict__ out, long ldo,   \
+      int M, int N, int K, int act, const float *__restrict__ ln_g, const float *__restrict__ ln_b, float ln_eps,     \
+      const float *__restrict__ pos, int pos_split
+#define ALM_GEMV_ARGS x, x2, n_split, ldx, W, bias, resid, ldr, out, ldo, M, N, K, act, ln_g, ln_b, ln_eps, pos, pos_split
+template <int MR, int NW>  // up to 32 rows
+__global__ void __launch_bounds__(128) gemv_rows_kernel(ALM_GEMV_PARAMS) {
+  gemv_rows_body<MR, NW>(ALM_GEMV_ARGS);
+}
+template <int NW>  // 64 rows: one CTA per SM by its shared memory anyway, so the 64 accumulators may take the registers
+__global__ void __launch_bounds__(128, 1) gemv_rows64_kernel(ALM_GEMV_PARAMS) {
+  gemv_rows_body<64, NW>(ALM_GEMV_ARGS);
+}
+#undef ALM_GEMV_PARAMS
+#undef ALM_GEMV_ARGS
 
 }  // namespace
 
@@ -707,28 +751,30 @@ void gemv_rows(Ctx* c, const float* x, const float* x2, int n_split, long ldx, c
                const float* ln_b, float ln_eps, const float* pos, int pos_split) {
   if (c->skipped(2)) return;
   ALM_REQUIRE(ln_g == nullptr || (K == 512 && ln_b != nullptr), ALM_ERR_INVALID, "gemv_rows: fused LayerNorm needs K == 512");
-  ALM_REQUIRE(M >= 1 && M <= 32 && K % 4 == 0 && ldx % 4 == 0 && K <= 2048 && n_split % 4 == 0 &&
+  ALM_REQUIRE(M >= 1 && M <= 64 && K % 4 == 0 && ldx % 4 == 0 && K <= 2048 && n_split % 4 == 0 &&
                   (K <= 512 || K % 512 == 0),
-              ALM_ERR_INVALID, "gemv_rows: M <= 32, K % 4 == 0, K <= 512 or a multiple of 512 up to 2048");
+              ALM_ERR_INVALID, "gemv_rows: M <= 64, K % 4 == 0, K <= 512 or a multiple of 512 up to 2048");
   const unsigned grid = static_cast<unsigned>((N + 3) / 4);
-  const size_t dyn = static_cast<size_t>(M) * (K <= 512 ? K : 2 * 512) * sizeof(float);
-#define ALM_GEMV(MRV, NWV)                                                                                         \
+  // staged rows: one K-wide buffer, or two chunk buffers (512 floats; 256 for the 64-row kernel) when K > 512
+  const size_t dyn = static_cast<size_t>(M) * (K <= 512 ? K : 2 * (M > 32 ? 256 : 512)) * sizeof(float);
+#define ALM_GEMV_K(KERNEL)                                                                                         \
   do {                                                                                                             \
     static alm::DeviceOnce attr;                                                                                   \
     if (attr.need()) {                                                                                              \
-      ALM_CHECK_CUDA(cudaFuncSetAttribute(gemv_rows_kernel<MRV, NWV>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                          128 * 1024));                                                            \
-      alm::pin_carveout(gemv_rows_kernel<MRV, NWV>);                                                               \
+      ALM_CHECK_CUDA(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 1024));       \
+      alm::pin_carveout(KERNEL);                                                                                   \
       attr.mark();                                                                                                 \
     }                                                                                                              \
-    gemv_rows_kernel<MRV, NWV><<<grid, 128, dyn, c->stream>>>(x, x2 ? x2 : x, n_split, ldx, W, bias, resid, ldr,   \
-                                                              out, ldo, M, N, K, act, ln_g, ln_b, ln_eps, pos,    \
-                                                              pos_split);                                         \
+    KERNEL<<<grid, 128, dyn, c->stream>>>(x, x2 ? x2 : x, n_split, ldx, W, bias, resid, ldr, out, ldo, M, N, K, act, \
+                                          ln_g, ln_b, ln_eps, pos, pos_split);                                     \
   } while (0)
+#define ALM_GEMV(MRV, NWV) ALM_GEMV_K((gemv_rows_kernel<MRV, NWV>))
   const int nw = K <= 512 ? 4 : 16;
   if (M <= 8) { if (nw == 4) ALM_GEMV(8, 4); else ALM_GEMV(8, 16); }
   else if (M <= 16) { if (nw == 4) ALM_GEMV(16, 4); else ALM_GEMV(16, 16); }
-  else { if (nw == 4) ALM_GEMV(32, 4); else ALM_GEMV(32, 16); }
+  else if (M <= 32) { if (nw == 4) ALM_GEMV(32, 4); else ALM_GEMV(32, 16); }
+  else { if (nw == 4) ALM_GEMV_K(gemv_rows64_kernel<4>); else ALM_GEMV_K(gemv_rows64_kernel<16>); }
+#undef ALM_GEMV_K
 #undef ALM_GEMV
   count_launch(c);
   check_launch("gemv_rows");

@@ -431,7 +431,7 @@ struct DecodeBufs {
   float *qk = nullptr, *v = nullptr, *scores = nullptr, *logits = nullptr, *qf = nullptr;
   float* qkv = nullptr;  // skinny path: fused [S,1536] q|k|v
   float *lnf = nullptr, *lnpf = nullptr, *attf = nullptr, *of = nullptr, *hidf = nullptr, *h0f = nullptr, *h1f = nullptr;
-  bool skinny = false;          // S <= 32 live sequences: all-fp32 SIMT GEMV path instead of tensor-core tiles
+  bool skinny = false;          // few live sequences: all-fp32 SIMT GEMV path instead of tensor-core tiles
   float* xq_partial = nullptr;  // fused single-query cross-attention: split partials + counters
   int* xq_counters = nullptr;
   int xq_splits = 1;
@@ -444,7 +444,9 @@ struct DecodeBufs {
   float* vc[4] = {nullptr, nullptr, nullptr, nullptr};
 };
 
-DecodeBufs alloc_decode(Ctx* c, OmniModel* m, int B, int Ncap, int Tmax) {
+// pt_loop: the point loop, whose Ncap sequences per image are the window prompts of the image.  It takes the exact-fp32
+// skinny path for at most 32 images and 64 rows (for one prompt per image: at most 32 images, as the other loops).
+DecodeBufs alloc_decode(Ctx* c, OmniModel* m, int B, int Ncap, int Tmax, bool pt_loop = false) {
   DecodeBufs d;
   d.S = B * Ncap; d.Tmax = Tmax; d.Ncap = Ncap;
   const size_t S = d.S;
@@ -462,7 +464,8 @@ DecodeBufs alloc_decode(Ctx* c, OmniModel* m, int B, int Ncap, int Tmax) {
   d.qk = c->ws.get<float>(S * 1024);
   d.v = c->ws.get<float>(S * 512);
   d.qf = c->ws.get<float>(S * 512);
-  d.skinny = (Ncap == 1 && d.S <= 32);
+  // several queries per image in the skinny path need the fused cross-attention (the unfused debug path is one query)
+  d.skinny = pt_loop ? (B <= 32 && d.S <= 64 && (Ncap == 1 || c->xattn_impl != 1)) : (Ncap == 1 && d.S <= 32);
   if (d.skinny) {
     d.lnf = c->ws.get<float>(S * 512); d.lnpf = c->ws.get<float>(S * 512); d.attf = c->ws.get<float>(S * 512);
     d.of = c->ws.get<float>(S * 512); d.hidf = c->ws.get<float>(S * 2048); d.h0f = c->ws.get<float>(S * 512);
@@ -531,8 +534,9 @@ void decoder_step(Ctx* c, OmniModel* m, int d, DecodeBufs& u, const int* tokens,
   embed_ln(c, tokens, tstride, u.tpos, S, m->word_emb, m->pos_emb[d], m->emb_norm.g, m->emb_norm.b, u.x, u.qpos);
   const float* qpos = u.qpos;
   if (u.skinny) {
-    // One live sequence per image and at most 32 of them: every linear is a skinny fp32 GEMV (exact fp32 weights,
-    // one warp per output column), no operand splitting, no tensor-core tile padding.
+    // At most 32 images and 64 live sequences (Ncap window prompts per image in the point loop, one otherwise): every
+    // linear is a skinny fp32 GEMV (exact fp32 weights, one warp per output column), no operand splitting, no tensor-core
+    // tile padding.  A row's arithmetic does not depend on how many rows share the launch.
     auto lin = [&](const float* x, int K, const Lin& w, int act, float* out, const float* resid) {
       gemv_rows(c, x, nullptr, 1 << 30, K, w.wf, w.b, resid, w.w.N, out, w.w.N, S, w.w.N, K, act);
     };
@@ -551,7 +555,7 @@ void decoder_step(Ctx* c, OmniModel* m, int d, DecodeBufs& u, const int* tokens,
         self_attn_step(c, u.qkv, u.qkv + 1024, u.kc[l], u.vc[l], S, u.tpos, u.Tmax, nullptr, nullptr, u.attf, 1536, 1536);
         lin(u.attf, 512, w.sa_out, ACT_NONE, u.x, u.x);
         lnlin(w.n2, qpos, 1 << 30, w.ca_q.wf, w.ca_q.b, 512, ACT_NONE, u.qf, 512);
-        fused_xattn(c, m, u, nullptr, nullptr, u.qf, img0, nimg, 1, dl, nullptr, nullptr, u.of);
+        fused_xattn(c, m, u, nullptr, nullptr, u.qf, img0, nimg, Ncap, dl, nullptr, nullptr, u.of);
         lin(u.of, 512, w.ca_out, ACT_NONE, u.x, u.x);
         lnlin(w.n3, nullptr, 0, w.l1.wf, w.l1.b, 2048, ACT_RELU, u.hidf, 2048);
         lin(u.hidf, 2048, w.l2, ACT_NONE, u.x, u.x);
@@ -578,7 +582,7 @@ void decoder_step(Ctx* c, OmniModel* m, int d, DecodeBufs& u, const int* tokens,
       const long koff = (static_cast<long>(img0) * 96 + dl * 8) * M * 64;
       const long voff = (static_cast<long>(img0) * 6144 + dl * 512) * Mpad;
       if (u.fused_xattn)
-        fused_xattn(c, m, u, nullptr, nullptr, u.qf, img0, nimg, 1, dl, nullptr, nullptr, u.of);
+        fused_xattn(c, m, u, nullptr, nullptr, u.qf, img0, nimg, Ncap, dl, nullptr, nullptr, u.of);
       else
         cross_attn_q1(c, u.qf, m->kc_hi + koff, m->kc_lo + koff, m->vt_hi + voff, m->vt_lo + voff,
                       m->kpm + static_cast<long>(img0) * M, nimg, M, Mpad, u.xq_partial, u.xq_counters, u.xq_splits, nullptr,
@@ -687,9 +691,8 @@ struct HeadArgs {
   int tstride = 0, n_prompt_m1 = 0;
   float* probs = nullptr;
   int pstride = 0;
-  int* finished = nullptr;
+  int* finished = nullptr;  // pt loop: per-sequence EOS state
   int* ntok = nullptr;
-  int seqs_per_image = 1;
   int nsoft = 0;  // logits entering the softmax (V, or V - vie_categories for the KIE poly/rec loops)
 };
 
@@ -703,14 +706,14 @@ void run_steps(Ctx* c, OmniModel* m, int d, DecodeBufs& u, const int* tokens, in
     decoder_step(c, m, d, u, tokens, tstride, img0, nimg, h.on);
     if (h.on)
       head_select(c, u.logits, u.S, m->V, h.nsoft ? h.nsoft : m->V, d, h.cfg, h.tokens, h.tstride, u.tpos, h.n_prompt_m1, h.probs, h.pstride,
-                  h.finished, h.ntok, h.seqs_per_image);
+                  h.finished, h.ntok);
     add_i32(c, u.tpos, 1);
   };
   if (!c->use_graphs || c->profile_gemm || c->gemm_impl != 0) {
     for (int i = 0; i < n; ++i) body();
     return;
   }
-  std::vector<long> key = {d, u.S, u.Ncap, u.Tmax, img0, nimg, m->M, h.on ? 1 : 0, c->nsplit,
+  std::vector<long> key = {d, u.S, u.Ncap, u.skinny ? 1 : 0, u.Tmax, img0, nimg, m->M, h.on ? 1 : 0, c->nsplit,
                            reinterpret_cast<long>(u.x), reinterpret_cast<long>(tokens), tstride,
                            reinterpret_cast<long>(h.probs), reinterpret_cast<long>(h.finished), h.n_prompt_m1,
                            reinterpret_cast<long>(m->kc_hi), reinterpret_cast<long>(u.kc[3]), h.cfg.pt_eos, h.cfg.num_bins,
@@ -745,21 +748,24 @@ void run_steps(Ctx* c, OmniModel* m, int d, DecodeBufs& u, const int* tokens, in
 
 }  // namespace
 
-// Greedy decoding of every encoded image.  Text spotting (transformer.py:234-286) and KIE (:143-217) share the
-// pt loop and the batched poly / rec loops; they differ in the pt step pattern (x, y[, class]), in which decoded
-// tokens form (x, y) instances and in the number of logits entering the poly / rec softmax.
-void omni_decode_impl(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_decode_cfg& cfg, bool kie,
+// Greedy decoding of every encoded image under R pt prompts each: B x R point sequences, sequence b * R + r being prompt r
+// of image b.  Text spotting (transformer.py:234-286) and KIE (:143-217) share the pt loop and the batched poly / rec
+// loops; they differ in the pt step pattern (x, y[, class]), in which decoded tokens form (x, y) instances and in the
+// number of logits entering the poly / rec softmax.  Outputs are per sequence; the poly / rec loops run per image over the
+// instances of all its prompts, concatenated in prompt order, so the K_c / V_c stream of an image serves every prompt.
+void omni_decode_impl(Ctx* c, const int64_t* prompts, int R, int n_prompt, const alm_decode_cfg& cfg, bool kie,
                       int32_t* n_tok_out, int64_t* pt_tok_out, float* pt_prob_out, int32_t* n_inst, int32_t* inst_pos,
                       int64_t* pt, int64_t* poly, int64_t* rec, float* rec_prob, bool points_only = false) {
   OmniModel* m = c->omni;
   ALM_REQUIRE(m && m->encoded, ALM_ERR_STATE, "alm_omni_decode before alm_omni_encode");
   ALM_REQUIRE(c->xattn_impl != 1 || m->vt_hi, ALM_ERR_STATE, "xattn_impl 1 must be set before alm_omni_encode");
   ALM_REQUIRE(n_prompt >= 1 && n_prompt <= 16, ALM_ERR_INVALID, "pt prompt length");
+  ALM_REQUIRE(R >= 1 && R <= 16, ALM_ERR_INVALID, "prompts per image must be 1..16");
   ALM_REQUIRE(cfg.pt_seq_length >= 1, ALM_ERR_INVALID, "pt_seq_length");
   // The reference default is --pt_seq_length 1024 (utils/parser.py:21) with a 5- or 7-token prompt: more steps than the
   // 1024-row position table (transformer.py:475) can serve.  It works because EOS ends the loop (:126) long before
   // step 1025 - n_prompt, where the embedding lookup (:312) would raise.  Same here: the loop is sized by the table,
-  // and an image that is still alive when the table is exhausted is an error, as in the reference.
+  // and a sequence that is still alive when the table is exhausted is an error, as in the reference.
   const int pt_steps = std::min(cfg.pt_seq_length, 1025 - n_prompt);
   const bool pt_clamped = pt_steps < cfg.pt_seq_length;
   ALM_REQUIRE(cfg.vie_categories == m->vie, ALM_ERR_INVALID, "vie_categories does not match the loaded checkpoint");
@@ -769,6 +775,7 @@ void omni_decode_impl(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_
   ALM_REQUIRE(points_only || cfg.max_instances >= (pt_steps / 2), ALM_ERR_INVALID, "max_instances < pt_seq_length / 2");
   ALM_REQUIRE(points_only || cfg.poly_length == 32, ALM_ERR_UNSUPPORTED, "polygon length is fixed at 32 (transformer.py:254)");
   const int B = m->B;
+  const int SP = B * R;  // point sequences
   Arena& ws = c->ws;
   ws.release(m->ws_mark);
   HeadCfg hc{cfg.num_bins, cfg.pt_eos, cfg.rec_eos, cfg.recog_pad, m->vie};
@@ -804,91 +811,92 @@ void omni_decode_impl(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_
   ALM_CHECK_CUDA(cudaEventRecord(c->ev_t[2], c->stream));
 
   // ------------------------------------------------------------------ pt loop (transformer.py:102-141)
+  // One prompt length for all sequences: the single device position counter and query position serve every row.
   const int Tpt = n_prompt + pt_steps;
-  int* pt_tok = ws.get<int>(static_cast<size_t>(B) * Tpt);
-  float* pt_prob = ws.get<float>(static_cast<size_t>(B) * pt_steps);
-  int* finished = ws.get<int>(B);
-  int* ntok = ws.get<int>(B);
+  int* pt_tok = ws.get<int>(static_cast<size_t>(SP) * Tpt);
+  float* pt_prob = ws.get<float>(static_cast<size_t>(SP) * pt_steps);
+  int* finished = ws.get<int>(SP);
+  int* ntok = ws.get<int>(SP);
   {
-    std::vector<int> h(static_cast<size_t>(B) * Tpt, 0);
-    for (int b = 0; b < B; ++b)
-      for (int i = 0; i < n_prompt; ++i) h[static_cast<size_t>(b) * Tpt + i] = static_cast<int>(pt_prompt[i]);
+    std::vector<int> h(static_cast<size_t>(SP) * Tpt, 0);
+    for (int s = 0; s < SP; ++s)
+      for (int i = 0; i < n_prompt; ++i)
+        h[static_cast<size_t>(s) * Tpt + i] = static_cast<int>(prompts[static_cast<size_t>(s) * n_prompt + i]);
     ALM_CHECK_CUDA(cudaMemcpyAsync(pt_tok, h.data(), h.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
     wait_stream(c, c->stream);  // h goes out of scope (this also waits for the encoder)
   }
-  fill_i32(c, finished, B, 0);
-  fill_i32(c, ntok, B, 0);
+  fill_i32(c, finished, SP, 0);
+  fill_i32(c, ntok, SP, 0);
   const size_t after_pt_tokens = ws.mark();
   {
-    DecodeBufs u = alloc_decode(c, m, B, 1, Tpt - 1);
+    DecodeBufs u = alloc_decode(c, m, B, R, Tpt - 1, true);
     fill_i32(c, u.tpos, 1, 0);
     HeadArgs off;
     run_steps(c, m, 0, u, pt_tok, Tpt, 0, B, n_prompt - 1, off);  // prompt tokens only fill the caches
     HeadArgs h;
     h.on = true; h.cfg = hc; h.tokens = pt_tok; h.tstride = Tpt; h.n_prompt_m1 = n_prompt - 1;
     h.probs = pt_prob; h.pstride = pt_steps;
-    h.finished = finished; h.ntok = ntok; h.seqs_per_image = 1;
-    std::vector<int> fin(B);
+    h.finished = finished; h.ntok = ntok;
+    std::vector<int> fin(SP);
     bool all_done = false;
     for (int done = 0; done < pt_steps && !all_done;) {
       const int chunk = std::min(16, pt_steps - done);
       run_steps(c, m, 0, u, pt_tok, Tpt, 0, B, chunk, h);
       done += chunk;
-      if (done < pt_steps || pt_clamped) {  // every image hit EOS?  (one small sync per 16 tokens)
+      if (done < pt_steps || pt_clamped) {  // every sequence hit EOS?  (one small sync per 16 tokens)
         wait_stream(c, c->stream);
-        ALM_CHECK_CUDA(cudaMemcpyAsync(fin.data(), finished, B * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        ALM_CHECK_CUDA(cudaMemcpyAsync(fin.data(), finished, SP * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
         ALM_CHECK_CUDA(cudaStreamSynchronize(c->stream));
         all_done = std::all_of(fin.begin(), fin.end(), [](int v) { return v != 0; });
       }
     }
     ALM_REQUIRE(!pt_clamped || all_done, ALM_ERR_INVALID,
-                "an image produced no EOS within the 1024-row position table (the reference raises at transformer.py:312)");
+                "a point sequence produced no EOS within the 1024-row position table (the reference raises at "
+                "transformer.py:312)");
   }
   ALM_CHECK_CUDA(cudaEventRecord(c->ev_t[3], c->stream));
   wait_stream(c, c->stream);
-  std::vector<int> h_ntok(B), h_tok(static_cast<size_t>(B) * Tpt);
-  std::vector<float> h_prob(static_cast<size_t>(B) * pt_steps);
-  ALM_CHECK_CUDA(cudaMemcpyAsync(h_ntok.data(), ntok, B * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  std::vector<int> h_ntok(SP), h_tok(static_cast<size_t>(SP) * Tpt);
+  std::vector<float> h_prob(static_cast<size_t>(SP) * pt_steps);
+  ALM_CHECK_CUDA(cudaMemcpyAsync(h_ntok.data(), ntok, SP * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
   ALM_CHECK_CUDA(cudaMemcpyAsync(h_tok.data(), pt_tok, h_tok.size() * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
   ALM_CHECK_CUDA(cudaMemcpyAsync(h_prob.data(), pt_prob, h_prob.size() * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
   ALM_CHECK_CUDA(cudaStreamSynchronize(c->stream));
   const int maxI = cfg.max_instances;
-  // which decoded tokens form (x, y) instances
-  std::vector<std::vector<int>> starts(B);
-  int Ncap = 0;
-  for (int b = 0; b < B; ++b) {
-    int len = h_ntok[b];
+  // which decoded tokens form (x, y) instances, per sequence
+  std::vector<std::vector<int>> starts(SP);
+  for (int s = 0; s < SP; ++s) {
+    int len = h_ntok[s];
     if (len % 2) --len;  // transformer.py:138-139 (applied in both modes by the reference)
-    const int* t = &h_tok[static_cast<size_t>(b) * Tpt + n_prompt];
+    const int* t = &h_tok[static_cast<size_t>(s) * Tpt + n_prompt];
     if (points_only) {  // the raw point sequence is the result (decode_pt_seq alone, transformer.py:102-141)
-      n_tok_out[b] = len;
+      n_tok_out[s] = len;
       for (int i = 0; i < len; ++i) {
-        pt_tok_out[static_cast<size_t>(b) * cfg.pt_seq_length + i] = t[i];
-        if (pt_prob_out) pt_prob_out[static_cast<size_t>(b) * cfg.pt_seq_length + i] = h_prob[static_cast<size_t>(b) * pt_steps + i];
+        pt_tok_out[static_cast<size_t>(s) * cfg.pt_seq_length + i] = t[i];
+        if (pt_prob_out) pt_prob_out[static_cast<size_t>(s) * cfg.pt_seq_length + i] = h_prob[static_cast<size_t>(s) * pt_steps + i];
       }
       continue;
     }
     if (!kie) {
-      for (int i = 0; i + 1 < len; i += 2) starts[b].push_back(i);
+      for (int i = 0; i + 1 < len; i += 2) starts[s].push_back(i);
     } else {
       for (int i = 0; i < len;) {  // the walk of decode_vie_pt_poly_rec_seq (transformer.py:148-215)
-        if (t[i] < cfg.num_bins && i + 1 <= len - 1 && t[i + 1] < cfg.num_bins) { starts[b].push_back(i); i += 2; }
+        if (t[i] < cfg.num_bins && i + 1 <= len - 1 && t[i + 1] < cfg.num_bins) { starts[s].push_back(i); i += 2; }
         else ++i;
       }
-      if (n_tok_out) n_tok_out[b] = len;
+      if (n_tok_out) n_tok_out[s] = len;
       for (int i = 0; i < len; ++i) {
-        pt_tok_out[static_cast<size_t>(b) * cfg.pt_seq_length + i] = t[i];
-        pt_prob_out[static_cast<size_t>(b) * cfg.pt_seq_length + i] = h_prob[static_cast<size_t>(b) * pt_steps + i];
+        pt_tok_out[static_cast<size_t>(s) * cfg.pt_seq_length + i] = t[i];
+        pt_prob_out[static_cast<size_t>(s) * cfg.pt_seq_length + i] = h_prob[static_cast<size_t>(s) * pt_steps + i];
       }
     }
-    n_inst[b] = static_cast<int>(starts[b].size());
-    ALM_REQUIRE(n_inst[b] <= maxI, ALM_ERR_INVALID, "decoded more points than max_instances");
-    Ncap = std::max(Ncap, n_inst[b]);
-    for (int n = 0; n < n_inst[b]; ++n) {
-      if (inst_pos) inst_pos[static_cast<size_t>(b) * maxI + n] = starts[b][n];
+    n_inst[s] = static_cast<int>(starts[s].size());
+    ALM_REQUIRE(n_inst[s] <= maxI, ALM_ERR_INVALID, "decoded more points than max_instances");
+    for (int n = 0; n < n_inst[s]; ++n) {
+      if (inst_pos) inst_pos[static_cast<size_t>(s) * maxI + n] = starts[s][n];
       if (pt) {
-        pt[(static_cast<size_t>(b) * maxI + n) * 2] = t[starts[b][n]];
-        pt[(static_cast<size_t>(b) * maxI + n) * 2 + 1] = t[starts[b][n] + 1];
+        pt[(static_cast<size_t>(s) * maxI + n) * 2] = t[starts[s][n]];
+        pt[(static_cast<size_t>(s) * maxI + n) * 2 + 1] = t[starts[s][n] + 1];
       }
     }
   }
@@ -897,6 +905,14 @@ void omni_decode_impl(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_
     ALM_CHECK_CUDA(cudaEventRecord(c->ev_t[4], c->stream));
     ws.release(m->ws_mark);
     return;
+  }
+  // the instances of image b: (sequence, instance) pairs of its prompts 0..R-1, in prompt order
+  std::vector<std::vector<std::pair<int, int>>> inst(B);
+  int Ncap = 0;
+  for (int b = 0; b < B; ++b) {
+    for (int r = 0; r < R; ++r)
+      for (int n = 0; n < n_inst[b * R + r]; ++n) inst[b].emplace_back(b * R + r, n);
+    Ncap = std::max(Ncap, static_cast<int>(inst[b].size()));
   }
   if (Ncap == 0) return;
 
@@ -920,8 +936,9 @@ void omni_decode_impl(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_
     for (int b = 0; b < B; ++b)
       for (int n = 0; n < Ncap; ++n) {
         int* row = &h_prompt[phase][(static_cast<size_t>(b) * Ncap + n) * T];
-        if (n < n_inst[b]) {
-          const int* t = &h_tok[static_cast<size_t>(b) * Tpt + n_prompt + starts[b][n]];
+        if (n < static_cast<int>(inst[b].size())) {
+          const int sq = inst[b][n].first;
+          const int* t = &h_tok[static_cast<size_t>(sq) * Tpt + n_prompt + starts[sq][inst[b][n].second]];
           row[0] = t[0]; row[1] = t[1];
         }
         row[2] = phase == 1 ? cfg.poly_sos : cfg.rec_sos;
@@ -944,7 +961,7 @@ void omni_decode_impl(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_
       run_steps(c, m, phase, u, toks[phase], T, 0, B, 2, off);
       HeadArgs h;
       h.on = true; h.cfg = hc; h.tokens = toks[phase]; h.tstride = T; h.n_prompt_m1 = 2; h.probs = prbs[phase];
-      h.pstride = len; h.seqs_per_image = Ncap;
+      h.pstride = len;
       h.nsoft = m->V - m->vie;  // logits[:, -1, :-vie_categories] (transformer.py:156,176)
       run_steps(c, m, phase, u, toks[phase], T, 0, B, len, h);
     }
@@ -968,10 +985,11 @@ void omni_decode_impl(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_
     ALM_CHECK_CUDA(cudaMemcpyAsync(hp.data(), prbs[phase], hp.size() * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     ALM_CHECK_CUDA(cudaStreamSynchronize(c->stream));
     for (int b = 0; b < B; ++b)
-      for (int n = 0; n < n_inst[b]; ++n) {
-        const size_t sq = static_cast<size_t>(b) * Ncap + n;
+      for (int j = 0; j < static_cast<int>(inst[b].size()); ++j) {  // scattered back per (image, prompt)
+        const size_t sq = static_cast<size_t>(b) * Ncap + j;
+        const size_t dst = static_cast<size_t>(inst[b][j].first) * maxI + inst[b][j].second;
         for (int k = 0; k < len; ++k) {
-          const size_t o = (static_cast<size_t>(b) * maxI + n) * len + k;
+          const size_t o = dst * len + k;
           if (phase == 1) poly[o] = hh[sq * T + 3 + k];
           else { rec[o] = hh[sq * T + 3 + k]; rec_prob[o] = hp[sq * len + k]; }
         }
@@ -980,22 +998,61 @@ void omni_decode_impl(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_
   ws.release(m->ws_mark);
 }
 
+namespace {
+// the single prompt of the classic entry points, broadcast to every encoded image
+std::vector<int64_t> broadcast_prompt(Ctx* c, const int64_t* pt_prompt, int n_prompt) {
+  ALM_REQUIRE(c->omni && c->omni->encoded, ALM_ERR_STATE, "alm_omni_decode before alm_omni_encode");
+  ALM_REQUIRE(n_prompt >= 1 && n_prompt <= 16, ALM_ERR_INVALID, "pt prompt length");
+  std::vector<int64_t> p(static_cast<size_t>(c->omni->B) * n_prompt);
+  for (size_t i = 0; i < p.size(); ++i) p[i] = pt_prompt[i % n_prompt];
+  return p;
+}
+
+// caller-supplied prompts [B][R][n_prompt] of the prompted entry points: every id is an embedding row
+void check_prompts(Ctx* c, const int64_t* prompts, int R, int n_prompt) {
+  OmniModel* m = c->omni;
+  ALM_REQUIRE(m && m->encoded, ALM_ERR_STATE, "alm_omni_decode_prompted before alm_omni_encode");
+  ALM_REQUIRE(m->vie == 0, ALM_ERR_UNSUPPORTED, "window-prompted decoding is text spotting only (not KIE checkpoints)");
+  ALM_REQUIRE(R >= 1 && R <= 16, ALM_ERR_INVALID, "prompts per image must be 1..16");
+  ALM_REQUIRE(n_prompt >= 1 && n_prompt <= 16, ALM_ERR_INVALID, "pt prompt length");
+  const size_t n = static_cast<size_t>(m->B) * R * n_prompt;
+  for (size_t i = 0; i < n; ++i)
+    ALM_REQUIRE(prompts[i] >= 0 && prompts[i] < m->V, ALM_ERR_INVALID, "prompt token id out of range [0, V)");
+}
+}  // namespace
+
 void omni_decode(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_decode_cfg& cfg, int32_t* n_inst,
                  int64_t* pt, int64_t* poly, int64_t* rec, float* rec_prob) {
-  omni_decode_impl(c, pt_prompt, n_prompt, cfg, false, nullptr, nullptr, nullptr, n_inst, nullptr, pt, poly, rec, rec_prob);
+  const std::vector<int64_t> p = broadcast_prompt(c, pt_prompt, n_prompt);
+  omni_decode_impl(c, p.data(), 1, n_prompt, cfg, false, nullptr, nullptr, nullptr, n_inst, nullptr, pt, poly, rec, rec_prob);
 }
 
 void omni_decode_kie(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_decode_cfg& cfg, int32_t* n_tok,
                      int64_t* pt_tokens, float* pt_probs, int32_t* n_inst, int32_t* inst_pos, int64_t* poly,
                      int64_t* rec, float* rec_prob) {
-  omni_decode_impl(c, pt_prompt, n_prompt, cfg, true, n_tok, pt_tokens, pt_probs, n_inst, inst_pos, nullptr, poly, rec,
+  const std::vector<int64_t> p = broadcast_prompt(c, pt_prompt, n_prompt);
+  omni_decode_impl(c, p.data(), 1, n_prompt, cfg, true, n_tok, pt_tokens, pt_probs, n_inst, inst_pos, nullptr, poly, rec,
                    rec_prob);
 }
 
 void omni_decode_points(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_decode_cfg& cfg, int32_t* n_tok,
                         int64_t* pt_tokens, float* pt_probs) {
-  omni_decode_impl(c, pt_prompt, n_prompt, cfg, c->omni && c->omni->vie > 0, n_tok, pt_tokens, pt_probs, nullptr, nullptr,
+  const std::vector<int64_t> p = broadcast_prompt(c, pt_prompt, n_prompt);
+  omni_decode_impl(c, p.data(), 1, n_prompt, cfg, c->omni->vie > 0, n_tok, pt_tokens, pt_probs, nullptr, nullptr,
                    nullptr, nullptr, nullptr, nullptr, true);
+}
+
+void omni_decode_prompted(Ctx* c, const int64_t* prompts, int R, int n_prompt, const alm_decode_cfg& cfg,
+                          int32_t* n_inst, int64_t* pt, int64_t* poly, int64_t* rec, float* rec_prob) {
+  check_prompts(c, prompts, R, n_prompt);
+  omni_decode_impl(c, prompts, R, n_prompt, cfg, false, nullptr, nullptr, nullptr, n_inst, nullptr, pt, poly, rec, rec_prob);
+}
+
+void omni_decode_points_prompted(Ctx* c, const int64_t* prompts, int R, int n_prompt, const alm_decode_cfg& cfg,
+                                 int32_t* n_tok, int64_t* pt_tokens, float* pt_probs) {
+  check_prompts(c, prompts, R, n_prompt);
+  omni_decode_impl(c, prompts, R, n_prompt, cfg, false, n_tok, pt_tokens, pt_probs, nullptr, nullptr, nullptr, nullptr,
+                   nullptr, nullptr, true);
 }
 
 // Teacher-forced logits for one image: every position of every sequence (Transformer.decode, :74-100).

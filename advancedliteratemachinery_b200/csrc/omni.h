@@ -15,7 +15,7 @@ struct LNW {
 struct Lin {
   SplitW w;
   float* b = nullptr;
-  float* wf = nullptr;  // exact fp32 [N,K] copy (decoder weights only): the skinny M <= 32 decode path
+  float* wf = nullptr;  // exact fp32 [N,K] copy (decoder weights only): the skinny M <= 64 decode path
 };
 
 struct SwinBlockW {
@@ -93,6 +93,11 @@ void omni_decode_kie(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_d
                      int64_t* rec, float* rec_prob);
 void omni_decode_points(Ctx* c, const int64_t* pt_prompt, int n_prompt, const alm_decode_cfg& cfg, int32_t* n_tok,
                         int64_t* pt_tokens, float* pt_probs);
+// R window prompts per image, prompts int64 [B][R][n_prompt] (text spotting): outputs per (image, prompt)
+void omni_decode_prompted(Ctx* c, const int64_t* prompts, int R, int n_prompt, const alm_decode_cfg& cfg,
+                          int32_t* n_inst, int64_t* pt, int64_t* poly, int64_t* rec, float* rec_prob);
+void omni_decode_points_prompted(Ctx* c, const int64_t* prompts, int R, int n_prompt, const alm_decode_cfg& cfg,
+                                 int32_t* n_tok, int64_t* pt_tokens, float* pt_probs);
 void omni_decode_logits(Ctx* c, int image, int kind, const int64_t* seq, int n_seq, int len, float* logits);
 
 // kernels (omni_kernels.cu)
@@ -108,8 +113,7 @@ void embed_ln(Ctx* c, const int* tokens, int tstride, const int* tptr, int S, co
 void self_attn_step(Ctx* c, const float* qk, const float* vnew, float* kc, float* vc, int S, const int* tptr, int Tmax,
                     bf16* out_hi, bf16* out_lo, float* out_f32 = nullptr, int ld_qk = 1024, int ld_v = 512);
 void head_select(Ctx* c, const float* logits, int S, int V, int nsoft, int phase, const HeadCfg& cfg, int* tokens,
-                 int tstride, const int* tptr, int n_prompt_m1, float* probs, int pstride, int* finished, int* ntok,
-                 int seqs_per_image);
+                 int tstride, const int* tptr, int n_prompt_m1, float* probs, int pstride, int* finished, int* ntok);
 void cross_attn_q1(Ctx* c, const float* q, const bf16* kc_hi, const bf16* kc_lo, const bf16* vt_hi, const bf16* vt_lo,
                    const uint8_t* kpm, int nimg, int M, int Mpad, float* partial, int* counters, int nsplit,
                    bf16* out_hi, bf16* out_lo, float* out_f32 = nullptr);

@@ -542,7 +542,7 @@ cross_attn_q1_kernel(const float* __restrict__ q, const bf16* __restrict__ kc_hi
 __global__ void __launch_bounds__(256)
 head_select_kernel(const float* __restrict__ logits, int V, int nsoft, int phase, HeadCfg cfg, int* __restrict__ tokens,
                    int tstride, const int* __restrict__ tptr, int n_prompt_m1, float* __restrict__ probs, int pstride,
-                   int* __restrict__ finished, int* __restrict__ ntok, int seqs_per_image) {
+                   int* __restrict__ finished, int* __restrict__ ntok) {
   __shared__ float redf[8];
   __shared__ int redi[8];
   const int s = blockIdx.x, t = threadIdx.x;
@@ -596,11 +596,10 @@ head_select_kernel(const float* __restrict__ logits, int V, int nsoft, int phase
     const float prob = expf(best - m) / tot;
     tokens[static_cast<long>(s) * tstride + tnext] = bi;
     if (probs) probs[static_cast<long>(s) * pstride + pidx] = prob;
-    if (finished) {  // pt loop: per-image EOS bookkeeping (transformer.py:126-127)
-      const int img = s / seqs_per_image;
-      if (!finished[img]) {
-        if (bi == cfg.pt_eos) finished[img] = 1;
-        else ntok[img] = gen_index + 1;
+    if (finished) {  // pt loop: per-sequence EOS bookkeeping (transformer.py:126-127; one window prompt each)
+      if (!finished[s]) {
+        if (bi == cfg.pt_eos) finished[s] = 1;
+        else ntok[s] = gen_index + 1;
       }
     }
   }
@@ -696,11 +695,10 @@ void self_attn_step(Ctx* c, const float* qk, const float* vnew, float* kc, float
   count_launch(c); check_launch("self_attn_step");
 }
 void head_select(Ctx* c, const float* logits, int S, int V, int nsoft, int phase, const HeadCfg& cfg, int* tokens,
-                 int tstride, const int* tptr, int n_prompt_m1, float* probs, int pstride, int* finished, int* ntok,
-                 int seqs_per_image) {
+                 int tstride, const int* tptr, int n_prompt_m1, float* probs, int pstride, int* finished, int* ntok) {
   ALM_PIN_CARVEOUT(head_select_kernel);
   head_select_kernel<<<S, 256, 0, c->stream>>>(logits, V, nsoft, phase, cfg, tokens, tstride, tptr, n_prompt_m1, probs,
-                                               pstride, finished, ntok, seqs_per_image);
+                                               pstride, finished, ntok);
   count_launch(c); check_launch("head_select");
 }
 void build_inst_prompts(Ctx* c, const int* pt_tokens, int pt_stride, int n_prompt, const int* ntok, int B, int Ncap,

@@ -67,6 +67,43 @@ class OmniVocab:
             p = [0, 0, self.num_bins - 1, self.num_bins - 1, self.pt_sos_index]
         return torch.tensor([p], dtype=torch.long)
 
+    def window_prompt(self, x0: int, y0: int, x1: int, y1: int, char_lo: int = 0,
+                      char_hi: Optional[int] = None) -> torch.Tensor:
+        """[1, n_prompt] pt prompt for a spatial window in bins and a character window in character indices (0 ..
+        len(chars)), the prompt layout the model is trained with (dataset/collate_fn.py:46-115; the decoder is meant to
+        emit the points with x0 < x <= x1, y0 < y <= y1 whose text lies in the character range).  The 5-token form
+        (no character window) when ``use_char_window_prompt`` is off."""
+        p = [int(x0), int(y0), int(x1), int(y1)]
+        if self.use_char_window_prompt:
+            hi = len(self.chars) if char_hi is None else int(char_hi)
+            p += [self.num_bins + int(char_lo), self.num_bins + hi]
+        return torch.tensor([p + [self.pt_sos_index]], dtype=torch.long)
+
+    def grid_prompts(self, nx: int, ny: int, char_window=None) -> torch.Tensor:
+        """[nx * ny, n_prompt] prompts of the nx x ny grid tiles of dataset/collate_fn.py:55-69 (same tile size
+        min(int(num_bins / n), num_bins - 1), same clamped ends, i over x outer, j over y inner).  char_window:
+        optional (char_lo, char_hi) shared by every tile."""
+        nb = self.num_bins
+        ix, iy = min(int(nb / nx), nb - 1), min(int(nb / ny), nb - 1)
+        lo, hi = char_window if char_window is not None else (0, None)
+        rows = []
+        for i in range(nx):
+            for j in range(ny):
+                x0, y0 = i * ix, j * iy
+                rows.append(self.window_prompt(x0, y0, min(x0 + ix, nb - 1), min(y0 + iy, nb - 1), lo, hi))
+        return torch.cat(rows, 0)
+
+
+def merge_window_outputs(outs):
+    """One reference-shaped output per page from its per-window outputs (prompt order, None windows skipped): the
+    instances of every window of the page, as ``postprocess`` / ``alm_post_omni_json`` take them; None when no window
+    decoded a point."""
+    live = [o for o in outs if o is not None]
+    if not live:
+        return None
+    return ([torch.cat([o[0][0] for o in live], 1), torch.cat([o[0][1] for o in live], 1),
+             torch.cat([o[0][2] for o in live], 1)], [torch.cat([o[1][0] for o in live], 0)])
+
 
 class OmniParserB200:
     """Inference-only stand-in for the reference ``OmniParser`` module (``--tfm_pre_norm --use_fpn``)."""
@@ -191,6 +228,63 @@ class OmniParserB200:
         self.ctx.check(self.lib.alm_omni_decode_points(self.ctx.h, prompt.data_ptr(), prompt.numel(), C.byref(cfg),
                                                        n_tok.ctypes.data, toks.ctypes.data, prob.ctypes.data))
         return [(torch.from_numpy(toks[b, :n_tok[b]].copy()), torch.from_numpy(prob[b, :n_tok[b]].copy())) for b in range(B)]
+
+    def _prompts(self, prompts: torch.Tensor):
+        """[R, L] (the same windows for every page) or [B, R, L] (per page) -> int64 [B, R, L] on the host."""
+        B, _, _ = self.memory_shape()
+        p = torch.as_tensor(prompts).to(torch.long).cpu()
+        if p.dim() == 2:
+            p = p.unsqueeze(0).expand(B, -1, -1)
+        if p.dim() != 3 or p.shape[0] != B:
+            raise ValueError(f'prompts must be [R, L] or [{B}, R, L], got {tuple(p.shape)}')
+        return p.contiguous()
+
+    def decode_prompted(self, prompts: torch.Tensor, merge: bool = False):
+        """Greedy decoding of every encoded page under R window prompts each (``OmniVocab.window_prompt`` /
+        ``grid_prompts``), over one encode.  prompts: [R, L] or [B, R, L].  Returns per page a list of R
+        reference-shaped outputs (None where a window decoded no point), each what ``decode`` returns for that page
+        under that prompt; with ``merge=True`` one output per page holding the instances of all its windows in prompt
+        order (``merge_window_outputs``)."""
+        v = self.vocab
+        p = self._prompts(prompts)
+        B, R, L = p.shape
+        maxi = max(1, v.pt_seq_length // 2)
+        n_inst = np.zeros((B, R), dtype=np.int32)
+        pt = np.zeros((B, R, maxi, 2), dtype=np.int64)
+        poly = np.zeros((B, R, maxi, 32), dtype=np.int64)
+        rec = np.zeros((B, R, maxi, v.rec_length), dtype=np.int64)
+        prob = np.zeros((B, R, maxi, v.rec_length), dtype=np.float32)
+        cfg = self._cfg(maxi)
+        self.ctx.check(self.lib.alm_omni_decode_prompted(self.ctx.h, p.data_ptr(), R, L, C.byref(cfg), n_inst.ctypes.data,
+                                                         pt.ctypes.data, poly.ctypes.data, rec.ctypes.data,
+                                                         prob.ctypes.data))
+        pages = []
+        for b in range(B):
+            outs = []
+            for r in range(R):
+                n = int(n_inst[b, r])
+                outs.append(None if n == 0 else
+                            ([torch.from_numpy(pt[b, r, :n].reshape(1, -1).copy()),
+                              torch.from_numpy(poly[b, r, :n].reshape(1, -1).copy()),
+                              torch.from_numpy(rec[b, r, :n][None].copy())],
+                             [torch.from_numpy(prob[b, r, :n].copy())]))
+            pages.append(merge_window_outputs(outs) if merge else outs)
+        return pages
+
+    def decode_points_prompted(self, prompts: torch.Tensor):
+        """`decode_pt_seq` alone under R window prompts per page: per page a list of R (tokens int64 [n], probs f32 [n])."""
+        v = self.vocab
+        p = self._prompts(prompts)
+        B, R, L = p.shape
+        P = v.pt_seq_length
+        n_tok = np.zeros((B, R), dtype=np.int32)
+        toks = np.zeros((B, R, P), dtype=np.int64)
+        prob = np.zeros((B, R, P), dtype=np.float32)
+        cfg = self._cfg(max(1, P // 2))
+        self.ctx.check(self.lib.alm_omni_decode_points_prompted(self.ctx.h, p.data_ptr(), R, L, C.byref(cfg),
+                                                                n_tok.ctypes.data, toks.ctypes.data, prob.ctypes.data))
+        return [[(torch.from_numpy(toks[b, r, :n_tok[b, r]].copy()), torch.from_numpy(prob[b, r, :n_tok[b, r]].copy()))
+                 for r in range(R)] for b in range(B)]
 
     def decode_kie(self, image_sizes, pt_prompt: Optional[torch.Tensor] = None):
         """KIE decoding of every encoded image (model/transformer.py:143-217): per image the reference's

@@ -220,6 +220,26 @@ ALM_API int alm_omni_decode(alm_ctx* ctx, const int64_t* pt_prompt, int n_prompt
 ALM_API int alm_omni_decode_points(alm_ctx* ctx, const int64_t* pt_prompt, int n_prompt, const alm_decode_cfg* cfg,
                                    int32_t* n_tok, int64_t* pt_tokens, float* pt_probs);
 
+/* Window-prompted text spotting: R pt prompts per encoded image, decoded over ONE encode (the encoder, FPN and
+ * cross-attention K/V of an image serve all its prompts).  A prompt is [x0, y0, x1, y1, char_lo, char_hi, pt_sos] (or
+ * the 5-token form without the character window): a spatial window in bins and a character window in class ids, as the
+ * model is trained (dataset/collate_fn.py:46-115).  Each (image b, prompt r) is exactly what alm_omni_decode returns
+ * for that image under that prompt: every prompt ends at its own EOS, and the polygon / recognition loops of an image
+ * take the points of all its prompts at once.  Tiling a page into R windows also lifts the 509-point cap of one point
+ * sequence (the 1024-row position table) to R x 509.
+ * prompts: int64 [B][R][n_prompt] (B = images of the last alm_omni_encode), 1 <= R <= 16, 1 <= n_prompt <= 16, every id
+ * in [0, V).  Outputs (host), per (image b, prompt r), max_inst = cfg->max_instances per prompt:
+ *   n_inst [B][R]; pt [B][R][max_inst][2]; poly [B][R][max_inst][32];
+ *   rec / rec_prob [B][R][max_inst][rec_length]
+ * Text-spotting checkpoints only: a KIE checkpoint returns ALM_ERR_UNSUPPORTED. */
+ALM_API int alm_omni_decode_prompted(alm_ctx* ctx, const int64_t* prompts, int R, int n_prompt, const alm_decode_cfg* cfg,
+                                     int32_t* n_inst, int64_t* pt, int64_t* poly, int64_t* rec, float* rec_prob);
+/* The point loop alone under R prompts per image: n_tok [B][R], pt_tokens / pt_probs [B][R][pt_seq_length] (pt_probs may
+ * be NULL), each (b, r) exactly what alm_omni_decode_points returns for that prompt. */
+ALM_API int alm_omni_decode_points_prompted(alm_ctx* ctx, const int64_t* prompts, int R, int n_prompt,
+                                            const alm_decode_cfg* cfg, int32_t* n_tok, int64_t* pt_tokens,
+                                            float* pt_probs);
+
 /* KIE variant (--infer_vie): replaces the eval branch with `decode_vie_pt_poly_rec_seq` (transformer.py:143-217,243-246).
  * The pt loop emits (x, y, class) triples (:117-123) with the class slot restricted to the last vie_categories
  * ids; every (x, y) pair found by the reference's walk (:148-210) gets a polygon and a transcription whose
