@@ -89,6 +89,15 @@ SIGNATURES = {
                                    C.c_int]),
     'alm_op_window_attention': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                           C.c_int, C.c_int, C.c_int]),
+    'alm_op_gemv': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_long, C.c_void_p, C.c_void_p, C.c_void_p,
+                              C.c_long, C.c_void_p, C.c_long, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                              C.c_float, C.c_void_p, C.c_int]),
+    'alm_op_self_attn_step': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                        C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    'alm_op_cross_attention': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                         C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    'alm_op_head_select': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(DecodeCfg),
+                                     C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     # test-time image pipeline
     'alm_pre_omni_plan': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int),
                                     C.POINTER(C.c_int)]),

@@ -7,6 +7,7 @@
 #include "mgp.h"
 #include "omni.h"
 #include "pre.h"
+#include "ptx.cuh"
 
 using namespace alm;
 
@@ -778,6 +779,183 @@ int alm_op_window_attention(alm_ctx* h, const float* qkv, const float* bias_tabl
     float* dd = c->ws.get<float>(dense.size());
     ALM_CHECK_CUDA(cudaMemcpyAsync(dd, dense.data(), dense.size() * 4, cudaMemcpyHostToDevice, c->stream));
     window_attention(c, qkv, C, heads, nWh, nWw, B, shift, nWh * 7, nWw * 7, dd, nullptr, nullptr, out);
+    ALM_CHECK_CUDA(cudaStreamSynchronize(c->stream));
+  });
+}
+
+int alm_op_gemv(alm_ctx* h, const float* x, const float* x2, int n_split, long ldx, const float* W, const float* bias,
+                const float* resid, long ldr, float* out, long ldo, int M, int N, int K, int act, const float* ln_g,
+                const float* ln_b, float ln_eps, const float* pos, int pos_split) {
+  return guarded(h, [&] {
+    ALM_REQUIRE(x && W && out && N > 0 && K > 0 && act >= 0 && act <= 2, ALM_ERR_INVALID, "alm_op_gemv arguments");
+    ALM_REQUIRE(ldx >= K && ldo >= N && (resid == nullptr || ldr >= N), ALM_ERR_INVALID, "alm_op_gemv strides");
+    gemv_rows(&h->c, x, x2, n_split, ldx, W, bias, resid, ldr, out, ldo, M, N, K, act, ln_g, ln_b, ln_eps, pos, pos_split);
+    ALM_CHECK_CUDA(cudaStreamSynchronize(h->c.stream));
+  });
+}
+
+int alm_op_self_attn_step(alm_ctx* h, const float* qk, int ld_qk, const float* vnew, int ld_v, float* kc, float* vc, int S,
+                          int t, int Tmax, float* out_f32, uint16_t* out_hi, uint16_t* out_lo) {
+  return guarded(h, [&] {
+    ALM_REQUIRE(qk && vnew && kc && vc && (out_f32 || out_hi) && S > 0, ALM_ERR_INVALID, "alm_op_self_attn_step arguments");
+    // the 1024-row position table bounds every decode loop; q / k rows are read as float4
+    ALM_REQUIRE(Tmax >= 1 && Tmax <= 1024 && t >= 0 && t < Tmax, ALM_ERR_INVALID, "alm_op_self_attn_step: 0 <= t < Tmax <= 1024");
+    ALM_REQUIRE(ld_qk >= 1024 && ld_qk % 4 == 0 && ld_v >= 512, ALM_ERR_INVALID, "alm_op_self_attn_step strides");
+    Ctx* c = &h->c;
+    c->ensure_ws();
+    ArenaScope arena_scope(c->ws);
+    int* tp = c->ws.get<int>(1);  // the kernels read the position from the device, as in a graph-replayed decode step
+    ALM_CHECK_CUDA(cudaMemcpyAsync(tp, &t, sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    self_attn_step(c, qk, vnew, kc, vc, S, tp, Tmax, reinterpret_cast<bf16*>(out_hi), reinterpret_cast<bf16*>(out_lo),
+                   out_f32, ld_qk, ld_v);
+    ALM_CHECK_CUDA(cudaStreamSynchronize(c->stream));
+  });
+}
+
+}  // extern "C"
+
+namespace {
+
+// [img][8][M][64] fp32 values of decoder-layer slot dl -> the feature-major V_c^T planes of the unfused path
+// ([img*6144 + dl*512 + h*64 + d][Mpad]); vt_* point at the first row of the slot, padding columns M..Mpad-1 are zero
+__global__ void op_vt_kernel(const float* __restrict__ v, int nimg, int M, int Mpad, bf16* __restrict__ vt_hi,
+                             bf16* __restrict__ vt_lo) {
+  const long i = static_cast<long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= static_cast<long>(nimg) * 512 * Mpad) return;
+  const int m = static_cast<int>(i % Mpad), f = static_cast<int>((i / Mpad) % 512), img = static_cast<int>(i / (512L * Mpad));
+  const float y = m < M ? v[((static_cast<long>(img) * 8 + (f >> 6)) * M + m) * 64 + (f & 63)] : 0.f;
+  const long o = (static_cast<long>(img) * 6144 + f) * Mpad + m;
+  split_bf16(y, vt_hi[o], vt_lo[o]);
+}
+
+__global__ void op_join_kernel(const bf16* __restrict__ hi, const bf16* __restrict__ lo, long n, float* __restrict__ out) {
+  const long i = static_cast<long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = __bfloat162float(hi[i]) + __bfloat162float(lo[i]);
+}
+
+}  // namespace
+
+extern "C" {
+
+int alm_op_cross_attention(alm_ctx* h, const float* q, const float* k, const float* v, const uint8_t* kpm, int B, int img0,
+                           int nimg, int Ncap, int M, int dl, int q_split, float* out) {
+  return guarded(h, [&] {
+    ALM_REQUIRE(q && k && v && out && B > 0 && nimg > 0 && img0 >= 0 && img0 + nimg <= B && Ncap > 0 && M > 0 && dl >= 0 &&
+                    dl < 12 && (q_split == 0 || q_split == 1),
+                ALM_ERR_INVALID, "alm_op_cross_attention arguments");
+    Ctx* c = &h->c;
+    const int impl = c->xattn_impl;
+    ALM_REQUIRE(impl != 1 || (Ncap == 1 && q_split == 0), ALM_ERR_UNSUPPORTED,
+                "alm_op_cross_attention: xattn_impl 1 runs the fused kernel for one fp32 query per image only");
+    c->ensure_ws();
+    ArenaScope arena_scope(c->ws);
+    // the K / V cache of alm_omni_encode: split bf16 [B*96 (image, decoder-layer slot, head)][M][64] per plane (and the
+    // feature-major V_c^T [B*6144][Mpad] for xattn_impl 1); every slice but (img0 .. img0+nimg-1, dl) holds NaN
+    const long slice = static_cast<long>(M) * 64, plane = static_cast<long>(B) * 96 * slice;
+    const int Mpad = (M + 7) & ~7;
+    const int nan2 = 0x7fc07fc0;  // two bf16 quiet NaNs
+    bf16* kv[4];
+    for (auto& p : kv) {
+      p = c->ws.get<bf16>(plane);
+      fill_i32(c, reinterpret_cast<int*>(p), plane / 2, nan2);
+    }
+    for (int i = img0; i < img0 + nimg; ++i) {
+      const long off = (static_cast<long>(i) * 96 + static_cast<long>(dl) * 8) * slice;
+      split_rows(c, k + i * 8 * slice, 64, 8L * M, 64, kv[0] + off, kv[1] + off, 64);
+      split_rows(c, v + i * 8 * slice, 64, 8L * M, 64, kv[2] + off, kv[3] + off, 64);
+    }
+    bf16 *vt_hi = nullptr, *vt_lo = nullptr;
+    if (impl == 1) {
+      const long vplane = static_cast<long>(B) * 6144 * Mpad;
+      vt_hi = c->ws.get<bf16>(vplane);
+      vt_lo = c->ws.get<bf16>(vplane);
+      fill_i32(c, reinterpret_cast<int*>(vt_hi), vplane / 2, nan2);
+      fill_i32(c, reinterpret_cast<int*>(vt_lo), vplane / 2, nan2);
+      const long voff = (static_cast<long>(img0) * 6144 + static_cast<long>(dl) * 512) * Mpad;
+      const long n = static_cast<long>(nimg) * 512 * Mpad;
+      op_vt_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->stream>>>(v + img0 * 8 * slice, nimg, M, Mpad,
+                                                                                  vt_hi + voff, vt_lo + voff);
+      check_launch("op_vt");
+    }
+    const long rows = static_cast<long>(nimg) * Ncap;
+    bf16 *q_hi = nullptr, *q_lo = nullptr;
+    if (q_split) {
+      q_hi = c->ws.get<bf16>(rows * 512);
+      q_lo = c->ws.get<bf16>(rows * 512);
+      split_rows(c, q, 512, rows, 512, q_hi, q_lo, 512);
+    }
+    const float* q_f32 = q_split ? nullptr : q;
+    // the decode loops take fp32 output only from fp32 queries on the <= 16-query path; otherwise the split pair
+    const bool f32_out = !q_split && Ncap <= 16;
+    bf16 *o_hi = nullptr, *o_lo = nullptr;
+    if (!f32_out) {
+      o_hi = c->ws.get<bf16>(rows * 512);
+      o_lo = c->ws.get<bf16>(rows * 512);
+    }
+    float* o_f32 = f32_out ? out : nullptr;
+    const uint8_t* kpm_i = kpm ? kpm + static_cast<long>(img0) * M : nullptr;
+    const long koff = (static_cast<long>(img0) * 96 + static_cast<long>(dl) * 8) * slice;
+    int* counters = nullptr;
+    int pairs = 0;
+    if (impl == 1) {  // alloc_decode + decoder_step for one query per image
+      const int ns = cross_attn_q1_splits(c, nimg, M);
+      float* partial = c->ws.get<float>(static_cast<size_t>(nimg) * 8 * ns * 66);
+      pairs = nimg * 8;
+      counters = c->ws.get<int>(pairs);
+      fill_i32(c, counters, pairs, 0);
+      const long voff = (static_cast<long>(img0) * 6144 + static_cast<long>(dl) * 512) * Mpad;
+      cross_attn_q1(c, q, kv[0] + koff, kv[1] + koff, vt_hi + voff, vt_lo + voff, kpm_i, nimg, M, Mpad, partial, counters,
+                    ns, o_hi, o_lo, o_f32);
+    } else {  // alloc_decode + fused_xattn
+      int grid = 1, parts = 1;
+      const bool tc = impl == 3 && Ncap > 16;
+      if (tc) cross_attn_tc_plan(c, nimg, Ncap, M, &grid, &parts, &pairs);
+      else if (impl == 2) cross_attn_tma_plan(c, nimg, Ncap, M, &grid, &parts, &pairs);
+      else cross_attn_mq_plan(c, nimg, Ncap, M, &grid, &parts, &pairs);
+      float* partial = c->ws.get<float>(cross_attn_mq_partial_floats(pairs, parts));
+      counters = c->ws.get<int>(pairs);
+      fill_i32(c, counters, pairs, 0);
+      const int z0 = static_cast<int>(img0 * 96 + dl * 8);
+      if (tc)
+        cross_attn_tc(c, q_hi, q_lo, q_f32, nimg, Ncap, kv[0], kv[1], kv[2], kv[3], static_cast<long>(B) * 96, z0, kpm_i, M,
+                      grid, parts, partial, counters, o_hi, o_lo, o_f32);
+      else if (impl == 2)
+        cross_attn_tma(c, q_hi, q_lo, q_f32, nimg, Ncap, kv[0], kv[1], kv[2], kv[3], static_cast<long>(B) * 96, z0, kpm_i, M,
+                       grid, parts, partial, counters, o_hi, o_lo, o_f32);
+      else
+        cross_attn_mq(c, q_hi, q_lo, q_f32, nimg, Ncap, kv[0] + koff, kv[1] + koff, kv[2] + koff, kv[3] + koff, kpm_i, M, grid,
+                      parts, partial, counters, o_hi, o_lo, o_f32);
+    }
+    if (!f32_out) {
+      const long n = rows * 512;
+      op_join_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, c->stream>>>(o_hi, o_lo, n, out);
+      check_launch("op_join");
+    }
+    // the merge counters reset themselves for the next launch (a captured decode step replays without re-zeroing them)
+    std::vector<int> cnt(pairs);
+    ALM_CHECK_CUDA(cudaMemcpyAsync(cnt.data(), counters, pairs * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    ALM_CHECK_CUDA(cudaStreamSynchronize(c->stream));
+    ALM_REQUIRE(std::all_of(cnt.begin(), cnt.end(), [](int x) { return x == 0; }), ALM_ERR_STATE,
+                "alm_op_cross_attention: merge counters were not reset by the kernel");
+  });
+}
+
+int alm_op_head_select(alm_ctx* h, const float* logits, int S, int V, int nsoft, int phase, const alm_decode_cfg* cfg, int t,
+                       int n_prompt_m1, int32_t* tokens, int tstride, float* probs, int pstride, int32_t* finished,
+                       int32_t* ntok) {
+  return guarded(h, [&] {
+    ALM_REQUIRE(logits && cfg && tokens && S > 0 && V > 0 && nsoft > 0 && nsoft <= V && phase >= 0 && phase <= 2,
+                ALM_ERR_INVALID, "alm_op_head_select arguments");
+    ALM_REQUIRE(t >= n_prompt_m1 && n_prompt_m1 >= 0 && t + 1 < tstride && (probs == nullptr || t - n_prompt_m1 < pstride),
+                ALM_ERR_INVALID, "alm_op_head_select: position / strides");
+    ALM_REQUIRE((finished == nullptr) == (ntok == nullptr), ALM_ERR_INVALID, "alm_op_head_select: finished and ntok go together");
+    Ctx* c = &h->c;
+    c->ensure_ws();
+    ArenaScope arena_scope(c->ws);
+    int* tp = c->ws.get<int>(1);
+    ALM_CHECK_CUDA(cudaMemcpyAsync(tp, &t, sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    const HeadCfg hc{cfg->num_bins, cfg->pt_eos, cfg->rec_eos, cfg->recog_pad, cfg->vie_categories};  // as omni.cu maps it
+    head_select(c, logits, S, V, nsoft, phase, hc, tokens, tstride, tp, n_prompt_m1, probs, pstride, finished, ntok);
     ALM_CHECK_CUDA(cudaStreamSynchronize(c->stream));
   });
 }

@@ -493,6 +493,12 @@ gemv_rows_body(const float* __restrict__ x, const float* __restrict__ x2, int n_
   const float* xin = (blockIdx.x * 4 < n_split) ? x : x2;  // columns [0, n_split) read x, the rest x2 (fused q|k|v)
   const uint32_t sbase = static_cast<uint32_t>(__cvta_generic_to_shared(sx));
   auto stage = [&](int chunk, int buf) {
+    // NC is sized for K = 2048: when K = 1024 or 1536 the trailing chunks lie past column K (KC divides K, so a chunk
+    // is either full or empty) -- they stage nothing, only commit their (empty) group so that the wait counts hold
+    if (NC > 1 && chunk * KC >= K) {
+      asm volatile("cp.async.commit_group;" ::: "memory");
+      return;
+    }
     const int k4 = KC >> 2;
     for (int i = threadIdx.x; i < M * k4; i += 128) {
       const int m = i / k4, c4 = i - m * k4;

@@ -274,6 +274,10 @@ void omni_encode(Ctx* c, const float* img, const uint8_t* mask, int B, int H, in
   if (c->xattn_impl == 1) {  // the unfused debug path multiplies P by a feature-major V_c^T
     m->vt_hi = ws.get<bf16>(static_cast<size_t>(B) * 6144 * m->Mpad);
     m->vt_lo = ws.get<bf16>(static_cast<size_t>(B) * 6144 * m->Mpad);
+    // the GEMM writes columns 0..M-1 only; cross_attn_q1 multiplies the padding columns M..Mpad-1 by p = 0, which stays
+    // 0 only if they hold finite values -- never whatever the arena held before
+    ALM_CHECK_CUDA(cudaMemsetAsync(m->vt_hi, 0, static_cast<size_t>(B) * 6144 * m->Mpad * sizeof(bf16), c->stream));
+    ALM_CHECK_CUDA(cudaMemsetAsync(m->vt_lo, 0, static_cast<size_t>(B) * 6144 * m->Mpad * sizeof(bf16), c->stream));
   }
   m->ws_mark = ws.mark();
 

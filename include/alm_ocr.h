@@ -290,6 +290,38 @@ ALM_API int alm_op_layernorm(alm_ctx* ctx, const float* x, const float* gamma, c
 ALM_API int alm_op_window_attention(alm_ctx* ctx, const float* qkv, const float* bias_table /*[169,heads]*/, float* out,
                             int B, int nWh, int nWw, int C, int heads, int shift);
 
+/* Kernels of the OmniParser decode step.  Every call synchronises before it returns. */
+/* Skinny exact-fp32 linear of the decode loops (M <= 64 rows, K <= 512 or K in {1024, 1536, 2048}):
+ *   out[m*ldo + n] = act(xin[m*ldx + 0..K) . W[n*K + 0..K) + bias[n]) (+ resid[m*ldr + n]),  act 0 none / 1 gelu / 2 relu
+ * with xin = x for the columns n < n_split and x2 (NULL: x) for the rest.  ln_g / ln_b non-NULL (K == 512): the rows are
+ * LayerNorm'd (eps ln_eps) first, and pos[0..512) is added to them for the columns n < pos_split.  bias / resid / pos may
+ * be NULL; n_split, pos_split and every stride are multiples of 4. */
+ALM_API int alm_op_gemv(alm_ctx* ctx, const float* x, const float* x2, int n_split, long ldx, const float* W, const float* bias,
+                        const float* resid, long ldr, float* out, long ldo, int M, int N, int K, int act, const float* ln_g,
+                        const float* ln_b, float ln_eps, const float* pos, int pos_split);
+/* Cached self-attention step at position t (host int, 0 <= t < Tmax <= 1024) for S sequences x 8 heads of width 64:
+ * appends k = qk[s*ld_qk + 512 .. 1024) and v = vnew[s*ld_v + 0 .. 512) as row t of kc / vc ([S][Tmax][512] fp32), then
+ * out[s] = softmax((q / 8) . kc[s][0..t]^T) vc[s][0..t] with q = qk[s*ld_qk + 0 .. 512).  out_f32 [S][512] and the split
+ * bf16 pair out_hi / out_lo (bits, [S][512]) may each be NULL.  The "sattn_wide" option picks the kernel as in the model. */
+ALM_API int alm_op_self_attn_step(alm_ctx* ctx, const float* qk, int ld_qk, const float* vnew, int ld_v, float* kc, float* vc,
+                                  int S, int t, int Tmax, float* out_f32, uint16_t* out_hi, uint16_t* out_lo);
+/* Decoder cross-attention of nimg images x Ncap queries against decoder-layer slot dl (0..11) of a K/V cache of B
+ * images: out[i*Ncap + n][h*64 + d] = softmax((q_n / 8) . K_{img0+i,h}^T, keys with kpm != 0 excluded) V_{img0+i,h}.
+ * q f32 [nimg*Ncap][512]; k, v f32 [B][8][M][64] (images img0 .. img0+nimg-1 are read); kpm u8 [B][M] or NULL.  The call
+ * lays the cache out as alm_omni_encode does, every slice it must not read filled with NaN, and runs the kernel the
+ * "xattn_impl" option selects for this shape, as the decode loops do.  q_split 1: the queries are split to bf16 hi / lo
+ * first (polygon / recognition loops).  out f32 [nimg*Ncap][512]. */
+ALM_API int alm_op_cross_attention(alm_ctx* ctx, const float* q, const float* k, const float* v, const uint8_t* kpm, int B,
+                                   int img0, int nimg, int Ncap, int M, int dl, int q_split, float* out);
+/* Greedy head step of the decode loops at position t: for each of S rows of logits [S][V], the top-1 of the candidate
+ * classes of `phase` (0 = point loop, whose mode follows the generated index t - n_prompt_m1; 1 = polygon; 2 =
+ * recognition), its softmax probability over the first nsoft logits; writes tokens[s*tstride + t + 1] and
+ * probs[s*pstride + t - n_prompt_m1] (probs may be NULL).  finished / ntok ([S] int32, both or neither): EOS bookkeeping
+ * of the point loop. */
+ALM_API int alm_op_head_select(alm_ctx* ctx, const float* logits, int S, int V, int nsoft, int phase, const alm_decode_cfg* cfg,
+                               int t, int n_prompt_m1, int32_t* tokens, int tstride, float* probs, int pstride,
+                               int32_t* finished, int32_t* ntok);
+
 /* ---- test-time image pipeline on the GPU (SURVEY 8f rank 1) ----------------------------------- */
 /* Replaces RandomResize([test_min_size], test_max_size) -> ToTensor -> Normalize -> nested_tensor_from_tensor_list
  * (OCR/OmniParser/dataset/__init__.py:109-113, dataset/transforms.py:249-298,312-322, utils/nested_tensor.py:37-54)
